@@ -29,6 +29,15 @@ per step.
   cpu_baseline / --impl reference   the oracle's reference-shaped restatement of the Go loop (1 thread —
              the reference's ApplyState is strictly sequential), bounded sample of the same workload;
              cpu_baseline.soa_scalar_1core: the same decisions over the SoA encoding (the generous CPU baseline)
+
+--dump-outputs DIR writes what the last timed step returned to its caller as float32 / float64 .npy files, so that
+two builds can be compared output for output (the inputs are a pure function of the arguments):
+  node_index   which nodes the other arrays hold: all of them, or a fixed seeded sample of DUMP_NODES sorted indices
+  next_state   next_state of those nodes
+  actions      action bits of those nodes
+  outcome      actuator outcome of those nodes (--pods only)
+  counters     every ust_counters field except `reserved`, in declaration order (hist[16] first)
+At N>1 each rank writes its own shard's files with a _rank<r> suffix and a proportionally smaller sample.
 """
 import argparse
 import ctypes as C
@@ -49,6 +58,7 @@ BYTES_PER_NODE = 16  # state 1 + flags 4 + pod_rev 4 + ds_idx 4 read, next_state
 SHARD_NODES = 10_000_000
 CPU_SAMPLE_NODES = 1_000_000
 L2_BYTES = 126 * 1024 * 1024
+DUMP_NODES = 1 << 21  # --dump-outputs: 8 + 4 + 4 (+ 4) bytes per sampled node, at most 40 MB in all
 
 
 def ncu_traffic():
@@ -270,6 +280,23 @@ def same_as_oracle(helpers, pol, soa, buf, pods=None):
     return bool(ok)
 
 
+def dump_outputs(out_dir, buf, cnt, rank, world):
+    """--dump-outputs: the outputs of one timed buffer set and the counters of the last call (module docstring)."""
+    n = int(buf["next"].shape[0])
+    m = min(n, DUMP_NODES // world)
+    idx = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, size=m, replace=False))
+    arrays = {"node_index": idx.astype(np.float64),
+              "next_state": buf["next"].cpu().numpy()[idx].astype(np.float32),
+              "actions": buf["actions"].cpu().numpy().view(np.uint16)[idx].astype(np.float32),
+              "counters": np.array(cnt["hist"] + [v for k, v in cnt.items() if k != "hist"], dtype=np.float64)}
+    if buf.get("outcome") is not None:
+        arrays["outcome"] = buf["outcome"].cpu().numpy()[idx].astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def print_stamps(ustlib, h):
     g = min(int(os.environ["UST_STAMPS"]), 148)
     st = (C.c_uint64 * (4 * g + 16))()
@@ -305,7 +332,13 @@ def main():
                          "ust_apply_state_packed (uint16 / int8: 8 instead of 13 bytes per node over PCIe)")
     ap.add_argument("--pods", action="store_true", help="tuning (with --quick): the C4 workload as the timed configuration")
     ap.add_argument("--no-by-config", action="store_true", help="skip the by_config legs (C2, C3_cut, C4, small)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ust: the reference run returns no outputs")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -396,10 +429,12 @@ def main():
     cnt = B.counters_dict()
     assert cnt["error_code"] == 0
     verified = None
+    last = (warmup + args.steps - 1) % SETS   # the buffer set of the last timed step
     if world == 1:
-        last = (warmup + args.steps - 1) % SETS
         verified = same_as_oracle(helpers, pol, soa, bufs[last], pods)
         assert verified, "timed outputs differ from the oracle"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bufs[last], cnt, rank, world)
 
     line = None
     if rank == 0:

@@ -53,11 +53,13 @@ def build_host_tests(root):
     bdir = os.path.join(tdir, "_build")
     os.makedirs(bdir, exist_ok=True)
     common = ["g++", "-O1", "-std=c++17", "-Wall", "-Wno-unused-variable", "-I" + root]
-    link = ["-L" + HERE, "-lust_host", "-lust", "-Wl,-rpath," + HERE]
+    # rpaths relative to the executables, so that a built tree still runs after it is copied or moved
+    link = ["-L" + HERE, "-lust_host", "-lust", "-Wl,-rpath,$ORIGIN/" + os.path.relpath(HERE, bdir)]
+    oracle = os.path.join(root, "oracle")
     srcs = [os.path.join(tdir, f) for f in os.listdir(tdir) if f.endswith((".cpp", ".hpp"))] + [HOST_OUT]
     out = []
     for name, extra in (("upgrade_state_test", []),
-                        ("host_logic_test", ["-L" + os.path.join(root, "oracle"), "-lust_oracle", "-Wl,-rpath," + os.path.join(root, "oracle")])):
+                        ("host_logic_test", ["-L" + oracle, "-lust_oracle", "-Wl,-rpath,$ORIGIN/" + os.path.relpath(oracle, bdir)])):
         exe = os.path.join(bdir, name)
         if not os.path.exists(exe) or any(os.path.getmtime(x) > os.path.getmtime(exe) for x in srcs):
             subprocess.check_call(common + [os.path.join(tdir, name + ".cpp"), "-o", exe] + link + extra)
