@@ -267,7 +267,8 @@ int ust_apply_state_packed(ust_handle* h, const ust_policy* policy, int64_t n_no
                            const int32_t* ds_rev, uint8_t* next_state, uint16_t* actions, uint8_t* actuator_outcome,
                            ust_counters* out);
 
-/* Delta form (SURVEY 8f.2): a successful ust_apply_state without pod lists leaves the uploaded snapshot resident on
+/* Delta form (SURVEY 8f.2): a ust_apply_state without pod lists that succeeds or ends in a reference-level abort
+ * (UST_ERR_REVISION_HASH, _MAX_UNAVAILABLE, _POD_DELETION_SPEC) leaves the uploaded snapshot resident on
  * the device. ust_apply_state_delta overwrites the n_changed nodes named by idx (distinct indices into that
  * snapshot) with freshly encoded values - what a reconcile that watches resourceVersions re-encodes - and evaluates
  * the whole snapshot again: same outputs and counters as ust_apply_state on the updated arrays, without

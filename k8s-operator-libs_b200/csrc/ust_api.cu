@@ -53,40 +53,64 @@ struct NcclApi {
 NcclApi g_nccl;
 std::mutex g_nccl_mu;
 
+// A device array that grows and is freed with its owner. Growing frees the old array at once: nothing may still use it.
 template <class T>
 struct DevBuf {
   T* p = nullptr;
   size_t cap = 0;  // elements
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+  ~DevBuf() { if (p) cudaFree(p); }
   cudaError_t reserve(size_t n) {
     if (n <= cap) return cudaSuccess;
     size_t want = cap ? cap : 1024;
     while (want < n) want += want / 2 + 1024;  // geometric growth
+    return resize(want);
+  }
+  // exactly n elements; the contents are not kept
+  cudaError_t resize(size_t n) {
     T* q = nullptr;
-    cudaError_t e = cudaMalloc(&q, want * sizeof(T));
+    cudaError_t e = cudaMalloc(&q, n * sizeof(T));
     if (e != cudaSuccess) return e;
     if (p) cudaFree(p);
     p = q;
-    cap = want;
+    cap = n;
     return cudaSuccess;
   }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
+
+// A CUDA resource of fixed size (device or pinned allocation, stream, event) that `Free` releases with its owner.
+// It reads as the raw handle.
+template <class T, auto Free>
+struct Owned {
+  T p{};
+  Owned() = default;
+  Owned(const Owned&) = delete;
+  Owned& operator=(const Owned&) = delete;
+  ~Owned() { if (p) Free(p); }
+  operator T() const { return p; }
+  T operator->() const { return p; }
+};
+template <class T> using DevPtr = Owned<T*, cudaFree>;
+template <class T> using PinnedPtr = Owned<T*, cudaFreeHost>;
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
 
 }  // namespace
 
 struct ust_handle {
   int device = -1;
-  cudaStream_t stream = nullptr;
-  cudaStream_t stream_d2h = nullptr;   // pipelined host path: downloads, kernels and uploads on three streams
-  cudaStream_t stream_h2d = nullptr;
-  cudaEvent_t seg_done[16] = {};
-  cudaEvent_t seg_up[16] = {};
-  cudaEvent_t d2h_done = nullptr;
+  Stream stream;
+  Stream stream_d2h;   // pipelined host path: downloads, kernels and uploads on three streams
+  Stream stream_h2d;
+  Event seg_done[16];
+  Event seg_up[16];
+  Event d2h_done;
   std::mutex mu;
   std::string err;
   int64_t launches = 0;
   int num_sms = 0;
-  size_t stream_smem = 0;   // dynamic shared memory of the streaming kernel (largest variant)
   bool ws_dirty = false;
   bool pdl = true;          // launch the kernels of a call with programmatic dependent launch (UST_PDL=0 turns it off: tuning)
   bool stamps = false;      // UST_STAMPS: per-CTA %globaltimer stamps (diagnostics)
@@ -97,29 +121,26 @@ struct ust_handle {
   struct Span { const char* p; size_t len; };
   Span prev_in[4] = {}, prev_out[3] = {};
   int64_t prev_n = -1;
-  bool chain_entry = false;     // set by ust_apply_state_device for the apply_device call it makes
   int64_t relaxed_calls = 0;   // diagnostics
   bool overlap_calls = true;  // UST_OVERLAP=0 turns the overlap of independent back-to-back calls off (tuning)
   cudaStream_t last_stream = nullptr;  // stream of the previous device-resident call (calls on another stream are ordered behind it)
   int64_t resident_n = -1;  // nodes of the snapshot the last ust_apply_state left in the staging arrays (-1 = none)
   int32_t resident_n_ds = 0;  // ... and the size of its DaemonSet table
-  ust_counters* hist_dev = nullptr;  // rollout simulation: one ust_counters per simulated reconcile
-  size_t hist_cap = 0;
+  DevBuf<ust_counters> hist;  // rollout simulation: one ust_counters per simulated reconcile
   int segments = 6;      // upload / compute / download pipeline depth of the host path (UST_SEGMENTS, tuning)
   bool no_hint = false;  // UST_NO_HINT=1 (tuning): every call speculates from the policy default, never from the previous call
 
-  UstWorkspace* ws = nullptr;
-  uint32_t* lut_dev = nullptr;      // UST_LUT_WORDS words
-  uint8_t* podlut_dev = nullptr;
-  uint32_t* lut_host = nullptr;     // pinned staging copy
-  uint8_t* podlut_host = nullptr;   // pinned
+  DevPtr<UstWorkspace> ws;
+  DevPtr<uint32_t> lut_dev;         // UST_LUT_WORDS words
+  DevPtr<uint8_t> podlut_dev;
+  PinnedPtr<uint32_t> lut_host;     // staging copy
+  PinnedPtr<uint8_t> podlut_host;
   ust_policy lut_policy;            // policy the device tables were built for
   bool lut_valid = false;
-  ust_counters* counters_dev = nullptr;
-  ust_counters* counters_host = nullptr;  // pinned
-  long long* xchg_dev = nullptr;
-  unsigned long long* ds_count_dev = nullptr;
-  size_t ds_count_cap = 0;
+  DevPtr<ust_counters> counters_dev;
+  PinnedPtr<ust_counters> counters_host;
+  DevPtr<long long> xchg_dev;
+  DevBuf<unsigned long long> ds_count;  // BuildState: pods per DaemonSet (zeroed whenever it is reallocated)
 
   // staging for the host-pointer API
   DevBuf<uint8_t> s_hot, s_next, s_outcome;
@@ -136,8 +157,8 @@ struct ust_handle {
   DevBuf<uint16_t> s_actions_prev, sp_actions;
   DevBuf<unsigned int> sp_blocks;
   DevBuf<long long> sp_idx;
-  long long* sp_count_dev = nullptr;
-  long long* sp_count_host = nullptr;  // pinned
+  DevPtr<long long> sp_count_dev;
+  PinnedPtr<long long> sp_count_host;
   bool outputs_resident = false;       // s_next / s_actions hold the outputs of the last call on the resident snapshot
   DevBuf<uint64_t> s_uid, s_dsuid;   // BuildState owner join: pod owner UIDs, DaemonSet UID hash table (+ s_dsorder: slot -> index)
   DevBuf<int32_t> s_dsorder;
@@ -151,7 +172,7 @@ struct ust_handle {
   int rank = 0, world = 1, comm_mode = 0;
   ncclComm_t comm = nullptr;
   // fused exchange: own mailbox + the peers' mailboxes mapped through CUDA IPC
-  UstMailbox* mbox_own = nullptr;
+  DevPtr<UstMailbox> mbox_own;
   UstMailbox* mbox[UST_MAX_WORLD] = {};
   bool mbox_ready = false;
   long long epoch = 0;
@@ -232,10 +253,25 @@ static int check_aligned(ust_handle* h, const void* p, const char* what) {
   return UST_OK;
 }
 
-static int fill_params(ust_handle* h, const ust_policy* policy, int64_t n, const uint8_t* state, const uint32_t* flags,
-                       const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds, const int32_t* ds_rev,
-                       const int32_t* pod_off, const uint16_t* pod_flags, uint8_t* next_state, uint16_t* actions,
-                       uint8_t* outcome, ust_counters* out_dev, UstParams* out, int* grid_out) {
+// Everything a call does before its streaming launches: order it behind the previous call, reset the workspace, build
+// the tables, fill the launch parameters, launch the pod summary (pod lists only) and give the call its collective
+// number and accumulator parity. The number is taken after the pod-summary launch: a call that fails before it leaves
+// epoch and call_seq as they were.
+static int begin_call(ust_handle* h, const ust_policy* policy, cudaStream_t st, int64_t n, const uint8_t* state,
+                      const uint32_t* flags, const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds, const int32_t* ds_rev,
+                      const int32_t* pod_off, const uint16_t* pod_flags, int64_t n_pods, uint8_t* next_state, uint16_t* actions,
+                      uint8_t* outcome, ust_counters* out_dev, UstParams* out, int* grid_out) {
+  // a handle's workspace, tables and counters serve one call at a time: a call on another stream than the previous
+  // one is ordered behind it (calls on the same stream are ordered by the stream)
+  if (h->last_stream && h->last_stream != st) UST_CUDA(h, cudaStreamSynchronize(h->last_stream));
+  h->last_stream = st;
+  if (h->ws_dirty) {
+    UST_CUDA(h, cudaMemsetAsync(h->ws, 0, sizeof(UstWorkspace), st));
+    h->ws_dirty = false;
+  }
+  int rc = ensure_tables(h, policy, st);
+  if (rc) return rc;
+
   const bool active = policy_active(policy);
   UstParams P;
   memset(&P, 0, sizeof(P));
@@ -293,6 +329,20 @@ static int fill_params(ust_handle* h, const ust_policy* policy, int64_t n, const
     cudaError_t ce = b.reserve((size_t)tiles + 1);
     if (ce != cudaSuccess) return h->fail(UST_ERR_CUDA, "cudaMalloc failed: %s", cudaGetErrorString(ce));
   }
+
+  h->ws_dirty = true;  // cleared again once every launch of this call has been enqueued successfully
+  if (P.eval_pods) {
+    // pod lists: one byte per node first (only the nodes whose actuator looks at its pods are read),
+    // then the ordinary streaming pass with that byte as a fifth input stream
+    UST_CUDA(h, h->s_podsum.reserve((size_t)n + 16));
+    P.podsum = h->s_podsum.p;
+    int e = ust_launch_pod_summary(n, P.active, P.hot, P.pod_off, P.pod_flags, n_pods, P.podlut, P.podsum, h->num_sms * 6, st);
+    if (e) return h->fail(UST_ERR_CUDA, "pod-summary kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+    h->launches += 1;
+  }
+  if (P.fused_exchange) P.epoch = ++h->epoch;  // collective call number: identical on every rank
+  P.parity = (int)(h->call_seq++ & 1u);
+  P.cand_tile = h->s_candtile[P.parity].p;
   *out = P;
   *grid_out = grid;
   return UST_OK;
@@ -320,14 +370,12 @@ static int check_pod_offsets_host(ust_handle* h, int64_t n, const int32_t* pod_o
   return UST_OK;
 }
 
-// core: everything device-resident, enqueue on `st`
-static int apply_device(ust_handle* h, const ust_policy* policy, int64_t n, const uint8_t* state, const uint32_t* flags,
-                        const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds, const int32_t* ds_rev,
+// core: everything device-resident, enqueue on `st`. `chain`: called by ust_apply_state_device, whose calls may
+// overlap the previous one.
+static int apply_device(ust_handle* h, bool chain, const ust_policy* policy, int64_t n, const uint8_t* state,
+                        const uint32_t* flags, const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds, const int32_t* ds_rev,
                         const int32_t* pod_off, const uint16_t* pod_flags, int64_t n_pods, uint8_t* next_state,
                         uint16_t* actions, uint8_t* outcome, ust_counters* out_dev, cudaStream_t st) {
-  const bool chain = h->chain_entry;  // called by ust_apply_state_device itself: the call may overlap the previous one
-  h->chain_entry = false;
-  if (!chain) h->prev_n = -1;
   if (n < 0) return h->fail(UST_ERR_NIL_STATE, "currentState should not be empty");
   if (n > 0 && (!state || !flags || !pod_rev || !ds_idx || !next_state || !actions))
     return h->fail(UST_ERR_NIL_STATE, "currentState should not be empty");
@@ -339,36 +387,11 @@ static int apply_device(ust_handle* h, const ust_policy* policy, int64_t n, cons
     if (ptrs[i]) { int rc = check_aligned(h, ptrs[i], names[i]); if (rc) return rc; }
   if (pod_off && pod_flags) { int rc = check_aligned(h, pod_flags, "pod_flags"); if (rc) return rc; }
   UST_CUDA(h, cudaSetDevice(h->device));
-  // a handle's workspace, tables and counters serve one call at a time: a call on another stream than the previous
-  // one is ordered behind it (calls on the same stream are ordered by the stream)
-  if (h->last_stream && h->last_stream != st) UST_CUDA(h, cudaStreamSynchronize(h->last_stream));
-  h->last_stream = st;
-  if (h->ws_dirty) {
-    UST_CUDA(h, cudaMemsetAsync(h->ws, 0, sizeof(UstWorkspace), st));
-    h->ws_dirty = false;
-  }
-  int rc = ensure_tables(h, policy, st);
-  if (rc) return rc;
-
   UstParams P;
   int grid = 0;
-  rc = fill_params(h, policy, n, state, flags, pod_rev, ds_idx, n_ds, ds_rev, pod_off, pod_flags, next_state, actions, outcome,
-                   out_dev, &P, &grid);
+  int rc = begin_call(h, policy, st, n, state, flags, pod_rev, ds_idx, n_ds, ds_rev, pod_off, pod_flags, n_pods, next_state,
+                      actions, outcome, out_dev, &P, &grid);
   if (rc) return rc;
-
-  h->ws_dirty = true;  // cleared again once every launch of this call has been enqueued successfully
-  if (P.eval_pods) {
-    // pod lists: one byte per node first (only the nodes whose actuator looks at its pods are read),
-    // then the ordinary streaming pass with that byte as a fifth input stream
-    UST_CUDA(h, h->s_podsum.reserve((size_t)n + 16));
-    P.podsum = h->s_podsum.p;
-    int e = ust_launch_pod_summary(n, P.active, P.hot, P.pod_off, P.pod_flags, n_pods, P.podlut, P.podsum, h->num_sms * 6, st);
-    if (e) return h->fail(UST_ERR_CUDA, "pod-summary kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-    h->launches += 1;
-  }
-  if (P.fused_exchange) P.epoch = ++h->epoch;  // collective call number: identical on every rank
-  P.parity = (int)(h->call_seq++ & 1u);
-  P.cand_tile = h->s_candtile[P.parity].p;
   // Independent back-to-back calls overlap: when the last thing enqueued on the handle's own stream is the previous
   // call's verification kernel and this call reads nothing that call writes and writes nothing that call reads or
   // writes, its streaming kernel does not wait for it (programmatic dependent launch without the initial wait: the
@@ -430,48 +453,109 @@ static int finish_with_counters(ust_handle* h, cudaStream_t st, ust_counters* ou
   return UST_OK;
 }
 
+static void drain_streams(ust_handle* h) {
+  if (h->stream_h2d) cudaStreamSynchronize(h->stream_h2d);
+  if (h->stream) cudaStreamSynchronize(h->stream);
+  if (h->stream_d2h) cudaStreamSynchronize(h->stream_d2h);
+}
+
 // Host-pointer entry points hand caller-owned buffers to asynchronous copies: whatever way such a call ends, nothing
 // of it may still be in flight when it returns (the caller may free or reuse the buffers).
 struct StreamDrain {
   ust_handle* h;
-  bool armed = true;
   explicit StreamDrain(ust_handle* hh) : h(hh) {}
-  ~StreamDrain() {
-    if (!armed) return;
-    if (h->stream_h2d) cudaStreamSynchronize(h->stream_h2d);
-    if (h->stream) cudaStreamSynchronize(h->stream);
-    if (h->stream_d2h) cudaStreamSynchronize(h->stream_d2h);
-  }
+  ~StreamDrain() { drain_streams(h); }
 };
 
-#pragma GCC visibility push(default)
+// Every entry point that takes a handle starts with UST_ENTER (after checks that touch nothing): one call at a time
+// per handle, and whatever the call enqueues sits between two device calls, which therefore keep the strict order.
+// Only ust_apply_state_device continues the overlap chain (chain = true).
+struct CallGuard {
+  std::lock_guard<std::mutex> lock;
+  CallGuard(ust_handle* h, bool chain) : lock(h->mu) { if (!chain) h->prev_n = -1; }
+};
+#define UST_ENTER(h)                          \
+  if (!(h)) return UST_ERR_INVALID_ARGUMENT; \
+  CallGuard call_guard_((h), false)
+
+// The resident snapshot: the staging arrays hold a snapshot that the delta calls, ust_fetch_outputs and the rollout
+// simulation may use. A call that stages into those arrays drops it first.
+static void drop_resident(ust_handle* h) {
+  h->resident_n = -1;
+  h->outputs_resident = false;
+}
+// Whether the snapshot a call has staged survives the call's return code: it does unless the call itself failed (CUDA,
+// the multi-GPU exchange). A reference-level abort (UST_ERR_REVISION_HASH, _MAX_UNAVAILABLE, _POD_DELETION_SPEC) is an
+// answer about the data and keeps it. Argument errors are returned before anything is staged or dropped: they leave the
+// previous snapshot as it was and never reach this rule.
+static bool snapshot_survives(int rc) { return rc != UST_ERR_CUDA && rc != UST_ERR_COMM; }
+static int keep_resident(ust_handle* h, int rc, int64_t n, int32_t n_ds) {
+  if (snapshot_survives(rc)) {
+    h->resident_n = n;
+    h->resident_n_ds = n_ds;
+    h->outputs_resident = true;
+  }
+  return rc;
+}
+
+// The dense outputs of nodes [n0, n0 + len) from the staging arrays to the caller's (actuator outcomes when asked for).
+static int download_outputs(ust_handle* h, int64_t n0, size_t len, uint8_t* next_state, uint16_t* actions, uint8_t* outcome,
+                            cudaStream_t st) {
+  if (!len) return UST_OK;
+  UST_CUDA(h, cudaMemcpyAsync(next_state + n0, h->s_next.p + n0, len, cudaMemcpyDeviceToHost, st));
+  UST_CUDA(h, cudaMemcpyAsync(actions + n0, h->s_actions.p + n0, len * 2, cudaMemcpyDeviceToHost, st));
+  if (outcome) UST_CUDA(h, cudaMemcpyAsync(outcome + n0, h->s_outcome.p + n0, len, cudaMemcpyDeviceToHost, st));
+  return UST_OK;
+}
+
+// The node columns of a host-staged ApplyState: wide (int32 pod_rev / ds_idx, as the kernels read them) or packed
+// (uint16 rev16 / int8 ds8: 3 instead of 8 bytes per node over PCIe, widened on the device).
+struct HostNodes {
+  ust_handle* h;
+  bool packed;
+  const uint8_t* state;
+  const uint32_t* flags;
+  const int32_t* pod_rev;
+  const int32_t* ds_idx;
+  const uint16_t* rev16;
+  const int8_t* ds8;
+
+  // copies nodes [n0, n0 + len) into the staging arrays
+  int upload_nodes(int64_t n0, size_t len, cudaStream_t st) const {
+    if (!len) return UST_OK;
+    UST_CUDA(h, cudaMemcpyAsync(h->s_hot.p + n0, state + n0, len, cudaMemcpyHostToDevice, st));
+    UST_CUDA(h, cudaMemcpyAsync(h->s_flags.p + n0, flags + n0, len * 4, cudaMemcpyHostToDevice, st));
+    if (packed) {
+      UST_CUDA(h, cudaMemcpyAsync(h->s_rev16.p + n0, rev16 + n0, len * 2, cudaMemcpyHostToDevice, st));
+      UST_CUDA(h, cudaMemcpyAsync(h->s_ds8.p + n0, ds8 + n0, len, cudaMemcpyHostToDevice, st));
+    } else {
+      UST_CUDA(h, cudaMemcpyAsync(h->s_rev.p + n0, pod_rev + n0, len * 4, cudaMemcpyHostToDevice, st));
+      UST_CUDA(h, cudaMemcpyAsync(h->s_ds.p + n0, ds_idx + n0, len * 4, cudaMemcpyHostToDevice, st));
+    }
+    return UST_OK;
+  }
+  // packed: widens the uploaded nodes [n0, n0 + len) into the int32 staging arrays
+  int widen_nodes(int64_t n0, size_t len, cudaStream_t st) const {
+    if (!packed || !len) return UST_OK;
+    int e = ust_launch_widen((long long)len, h->s_rev16.p + n0, h->s_ds8.p + n0, h->s_rev.p + n0, h->s_ds.p + n0, 4 * h->num_sms, st);
+    if (e) return h->fail(UST_ERR_CUDA, "widen kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+    h->launches += 1;
+    return UST_OK;
+  }
+};
 
 // Pipelined host path: the snapshot is cut into segments of whole tiles; segment s+1 uploads while segment
 // s streams through the kernel and segment s-1's results download (PCIe is full duplex). The streaming pass
 // is speculative, so a segment's outputs are final unless the end-of-call verification had to redo tiles —
 // then (rare) the outputs are downloaded again.
-static int apply_pipelined(ust_handle* h, const ust_policy* policy, int64_t n, const uint8_t* state, const uint32_t* flags,
-                           const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds, uint8_t* next_state,
-                           uint16_t* actions, uint8_t* outcome, ust_counters* out, const uint16_t* rev16 = nullptr,
-                           const int8_t* ds8 = nullptr) {
+static int apply_pipelined(ust_handle* h, const HostNodes& nodes, const ust_policy* policy, int64_t n, int32_t n_ds,
+                           uint8_t* next_state, uint16_t* actions, uint8_t* outcome, ust_counters* out) {
   cudaStream_t up = h->stream, down = h->stream_d2h, h2d = h->stream_h2d;  // up = compute stream of the call
-  if (h->last_stream && h->last_stream != up) UST_CUDA(h, cudaStreamSynchronize(h->last_stream));
-  h->last_stream = up;
-  if (h->ws_dirty) {
-    UST_CUDA(h, cudaMemsetAsync(h->ws, 0, sizeof(UstWorkspace), up));
-    h->ws_dirty = false;
-  }
-  int rc = ensure_tables(h, policy, up);
-  if (rc) return rc;
   UstParams P;
   int grid = 0;
-  rc = fill_params(h, policy, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p, nullptr, nullptr,
-                   h->s_next.p, h->s_actions.p, outcome ? h->s_outcome.p : nullptr, nullptr, &P, &grid);
+  int rc = begin_call(h, policy, up, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p, nullptr, nullptr, 0,
+                      h->s_next.p, h->s_actions.p, outcome ? h->s_outcome.p : nullptr, nullptr, &P, &grid);
   if (rc) return rc;
-  if (P.fused_exchange) P.epoch = ++h->epoch;
-  P.parity = (int)(h->call_seq++ & 1u);
-  P.cand_tile = h->s_candtile[P.parity].p;
-  h->prev_n = -1;
   const int tiles = P.n_tiles;
   // Segments: the uploads are the critical path (PCIe), every segment costs ~25 us of copy-engine turnarounds (measured:
   // 6 / 8 / 12 / 16 segments -> 1.80 / 1.87 / 1.95 / 2.06 ms at 10 M nodes), and what follows the last upload - its
@@ -479,10 +563,6 @@ static int apply_pipelined(ust_handle* h, const ust_policy* policy, int64_t n, c
   const int kSegments = h->segments;  // <= UST_MAX_SEGMENTS: one ticket counter and one event pair per streaming launch
   const int last_tiles = (kSegments > 1 && tiles >= 64) ? tiles / 16 : 0;
   const int per = last_tiles ? (tiles - last_tiles + kSegments - 2) / (kSegments - 1) : (tiles + kSegments - 1) / kSegments;
-  h->ws_dirty = true;
-  const bool dbg = getenv("UST_DEBUG_PIPE") != nullptr;
-  cudaEvent_t ev[4];
-  if (dbg) { for (auto& e : ev) cudaEventCreate(&e); cudaEventRecord(ev[0], up); }
   // uploads start once the compute stream has reached this call (tables, DaemonSet table, previous call's reads)
   UST_CUDA(h, cudaEventRecord(h->d2h_done, up));
   UST_CUDA(h, cudaStreamWaitEvent(h2d, h->d2h_done, 0));
@@ -491,24 +571,10 @@ static int apply_pipelined(ust_handle* h, const ust_policy* policy, int64_t n, c
     c1 = c0 + per < tiles - last_tiles ? c0 + per : (c0 < tiles - last_tiles ? tiles - last_tiles : tiles);
     const int64_t n0 = (int64_t)c0 * P.tile_nodes, n1 = c1 == tiles ? n : (int64_t)c1 * P.tile_nodes;
     const size_t len = (size_t)(n1 - n0);
-    if (len) {
-      UST_CUDA(h, cudaMemcpyAsync(h->s_hot.p + n0, state + n0, len, cudaMemcpyHostToDevice, h2d));
-      UST_CUDA(h, cudaMemcpyAsync(h->s_flags.p + n0, flags + n0, len * 4, cudaMemcpyHostToDevice, h2d));
-      if (rev16) {  // packed host format: 3 instead of 8 bytes per node over PCIe, widened on the device
-        UST_CUDA(h, cudaMemcpyAsync(h->s_rev16.p + n0, rev16 + n0, len * 2, cudaMemcpyHostToDevice, h2d));
-        UST_CUDA(h, cudaMemcpyAsync(h->s_ds8.p + n0, ds8 + n0, len, cudaMemcpyHostToDevice, h2d));
-      } else {
-        UST_CUDA(h, cudaMemcpyAsync(h->s_rev.p + n0, pod_rev + n0, len * 4, cudaMemcpyHostToDevice, h2d));
-        UST_CUDA(h, cudaMemcpyAsync(h->s_ds.p + n0, ds_idx + n0, len * 4, cudaMemcpyHostToDevice, h2d));
-      }
-    }
+    if ((rc = nodes.upload_nodes(n0, len, h2d))) return rc;
     UST_CUDA(h, cudaEventRecord(h->seg_up[seg], h2d));
     UST_CUDA(h, cudaStreamWaitEvent(up, h->seg_up[seg], 0));
-    if (rev16 && len) {
-      int we = ust_launch_widen((long long)len, h->s_rev16.p + n0, h->s_ds8.p + n0, h->s_rev.p + n0, h->s_ds.p + n0, 4 * h->num_sms, up);
-      if (we) return h->fail(UST_ERR_CUDA, "widen kernel launch failed: %s", cudaGetErrorString((cudaError_t)we));
-      h->launches += 1;
-    }
+    if ((rc = nodes.widen_nodes(n0, len, up))) return rc;
     UstParams Ps = P;
     Ps.tile_begin = c0;
     Ps.tile_end = c1;
@@ -522,37 +588,89 @@ static int apply_pipelined(ust_handle* h, const ust_policy* policy, int64_t n, c
     h->launches += 1;
     UST_CUDA(h, cudaEventRecord(h->seg_done[seg], up));
     UST_CUDA(h, cudaStreamWaitEvent(down, h->seg_done[seg], 0));
-    if (len) {
-      UST_CUDA(h, cudaMemcpyAsync(next_state + n0, h->s_next.p + n0, len, cudaMemcpyDeviceToHost, down));
-      UST_CUDA(h, cudaMemcpyAsync(actions + n0, h->s_actions.p + n0, len * 2, cudaMemcpyDeviceToHost, down));
-      if (outcome) UST_CUDA(h, cudaMemcpyAsync(outcome + n0, h->s_outcome.p + n0, len, cudaMemcpyDeviceToHost, down));
-    }
+    if ((rc = download_outputs(h, n0, len, next_state, actions, outcome, down))) return rc;
   }
-  if (dbg) { cudaEventRecord(ev[1], up); }
   rc = launch_verify(h, P, up, false);
   if (rc) return rc;
   h->ws_dirty = false;
   UST_CUDA(h, cudaMemcpyAsync(h->counters_host, h->counters_dev, sizeof(ust_counters), cudaMemcpyDeviceToHost, up));
-  if (dbg) { cudaEventRecord(ev[2], up); cudaEventRecord(ev[3], down); }
   cudaError_t ce = cudaStreamSynchronize(up);
   if (ce == cudaSuccess) ce = cudaStreamSynchronize(down);
-  if (dbg) {
-    float a, b, c;
-    cudaEventElapsedTime(&a, ev[0], ev[1]); cudaEventElapsedTime(&b, ev[0], ev[2]); cudaEventElapsedTime(&c, ev[0], ev[3]);
-    fprintf(stderr, "[ust pipe] uploads+stream kernels done %.3f ms, verify+counters %.3f ms, downloads done %.3f ms\n", a, b, c);
-    for (auto& e2 : ev) cudaEventDestroy(e2);
-  }
   if (ce != cudaSuccess) {
     h->ws_dirty = true;
     return h->fail(UST_ERR_CUDA, "kernel execution failed: %s", cudaGetErrorString(ce));
   }
-  if (h->counters_host->reserved[0] != 0) {  // the verification redid tiles: fetch the final outputs
-    UST_CUDA(h, cudaMemcpyAsync(next_state, h->s_next.p, (size_t)n, cudaMemcpyDeviceToHost, up));
-    UST_CUDA(h, cudaMemcpyAsync(actions, h->s_actions.p, (size_t)n * 2, cudaMemcpyDeviceToHost, up));
-    if (outcome) UST_CUDA(h, cudaMemcpyAsync(outcome, h->s_outcome.p, (size_t)n, cudaMemcpyDeviceToHost, up));
-  }
-  return finish_with_counters(h, up, out, h->counters_host->reserved[0] == 0);
+  const bool redone = h->counters_host->reserved[0] != 0;  // the verification redid tiles: fetch the final outputs
+  if (redone && (rc = download_outputs(h, 0, (size_t)n, next_state, actions, outcome, up))) return rc;
+  return finish_with_counters(h, up, out, !redone);
 }
+
+// ust_apply_state and ust_apply_state_packed, once their arguments have been checked: stage the snapshot, evaluate it,
+// return the outputs. Without pod lists the staged snapshot stays resident (see keep_resident); with pod lists it does
+// not, because the calls on the resident snapshot evaluate no pod lists.
+static int apply_host(ust_handle* h, const ust_policy* policy, int64_t n, const HostNodes& nodes, int32_t n_ds,
+                      const int32_t* ds_rev, const ust_pods* pods, uint8_t* next_state, uint16_t* actions, uint8_t* outcome,
+                      ust_counters* out) {
+  UST_CUDA(h, cudaSetDevice(h->device));
+  StreamDrain drain(h);
+  cudaStream_t st = h->stream;
+  const size_t N = (size_t)n;
+  UST_CUDA(h, h->s_hot.reserve(N + 16));
+  UST_CUDA(h, h->s_flags.reserve(N + 4));
+  UST_CUDA(h, h->s_rev.reserve(N + 4));
+  UST_CUDA(h, h->s_ds.reserve(N + 4));
+  if (nodes.packed) {
+    UST_CUDA(h, h->s_rev16.reserve(N + 8));
+    UST_CUDA(h, h->s_ds8.reserve(N + 16));
+  }
+  UST_CUDA(h, h->s_next.reserve(N + 16));
+  UST_CUDA(h, h->s_actions.reserve(N + 8));
+  UST_CUDA(h, h->s_dsrev.reserve((size_t)n_ds + 1));
+  if (outcome) UST_CUDA(h, h->s_outcome.reserve(N + 16));
+  if (pods) {
+    UST_CUDA(h, h->s_podoff.reserve(N + 1));
+    UST_CUDA(h, h->s_podflags.reserve((size_t)pods->n_pods + 8));
+  }
+  if (n_ds) UST_CUDA(h, cudaMemcpyAsync(h->s_dsrev.p, ds_rev, (size_t)n_ds * 4, cudaMemcpyHostToDevice, st));
+  drop_resident(h);
+  if (!pods && n >= (1 << 19))
+    return keep_resident(h, apply_pipelined(h, nodes, policy, n, n_ds, next_state, actions, outcome, out), n, n_ds);
+  int rc = nodes.upload_nodes(0, N, st);
+  if (rc) return rc;
+  if (pods) {
+    UST_CUDA(h, cudaMemcpyAsync(h->s_podoff.p, pods->pod_off, (N + 1) * 4, cudaMemcpyHostToDevice, st));
+    if (pods->n_pods) UST_CUDA(h, cudaMemcpyAsync(h->s_podflags.p, pods->pod_flags, (size_t)pods->n_pods * 2, cudaMemcpyHostToDevice, st));
+  }
+  if ((rc = nodes.widen_nodes(0, N, st))) return rc;
+  rc = apply_device(h, false, policy, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p,
+                    pods ? h->s_podoff.p : nullptr, pods ? h->s_podflags.p : nullptr, pods ? pods->n_pods : 0, h->s_next.p,
+                    h->s_actions.p, outcome ? h->s_outcome.p : nullptr, nullptr, st);
+  if (rc) return rc;
+  if ((rc = download_outputs(h, 0, N, next_state, actions, outcome, st))) return rc;
+  rc = finish_with_counters(h, st, out);
+  return pods ? rc : keep_resident(h, rc, n, n_ds);
+}
+
+// BuildState staging shared by both forms: pod columns, DaemonSet sizes, per-DaemonSet counters and a clean workspace
+static int stage_build_state(ust_handle* h, size_t n_pods, int32_t n_ds, cudaStream_t st) {
+  UST_CUDA(h, h->s_hot.reserve(n_pods + 16));
+  UST_CUDA(h, h->s_ds.reserve(n_pods + 4));
+  UST_CUDA(h, h->s_dsdesired.reserve((size_t)n_ds + 1));
+  if ((size_t)n_ds + 1 > h->ds_count.cap) {
+    UST_CUDA(h, h->ds_count.resize((size_t)n_ds + 64));
+    UST_CUDA(h, cudaMemsetAsync(h->ds_count.p, 0, h->ds_count.cap * sizeof(unsigned long long), st));
+  }
+  if (h->ws_dirty) { UST_CUDA(h, cudaMemsetAsync(h->ws, 0, sizeof(UstWorkspace), st)); h->ws_dirty = false; }
+  return UST_OK;
+}
+static int build_state_grid(const ust_handle* h, int64_t n_pods) {
+  int64_t grid = (n_pods + 1023) / 1024;  // 256 threads x 4 pods per iteration
+  if (grid < 1) grid = 1;
+  if (grid > 8 * h->num_sms) grid = 8 * h->num_sms;
+  return (int)grid;
+}
+
+#pragma GCC visibility push(default)
 
 extern "C" {
 
@@ -587,31 +705,32 @@ int ust_create(ust_handle** out, int device) {
     return UST_ERR_CUDA;
   };
   if ((e = cudaSetDevice(device)) != cudaSuccess) return bail("cudaSetDevice", e);
-  if ((e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
-  if ((e = cudaStreamCreateWithFlags(&h->stream_d2h, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
-  if ((e = cudaStreamCreateWithFlags(&h->stream_h2d, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
+  if ((e = cudaStreamCreateWithFlags(&h->stream.p, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
+  if ((e = cudaStreamCreateWithFlags(&h->stream_d2h.p, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
+  if ((e = cudaStreamCreateWithFlags(&h->stream_h2d.p, cudaStreamNonBlocking)) != cudaSuccess) return bail("cudaStreamCreate", e);
   for (auto& ev : h->seg_up)
-    if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+    if ((e = cudaEventCreateWithFlags(&ev.p, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
   for (auto& ev : h->seg_done)
-    if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
-  if ((e = cudaEventCreateWithFlags(&h->d2h_done, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
-  if ((e = cudaMalloc(&h->ws, sizeof(UstWorkspace))) != cudaSuccess) return bail("cudaMalloc", e);
+    if ((e = cudaEventCreateWithFlags(&ev.p, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+  if ((e = cudaEventCreateWithFlags(&h->d2h_done.p, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+  if ((e = cudaMalloc(&h->ws.p, sizeof(UstWorkspace))) != cudaSuccess) return bail("cudaMalloc", e);
   if ((e = cudaMemset(h->ws, 0, sizeof(UstWorkspace))) != cudaSuccess) return bail("cudaMemset", e);
-  if ((e = cudaMalloc(&h->lut_dev, UST_LUT_WORDS * sizeof(uint32_t))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMalloc(&h->podlut_dev, UST_PODLUT_ENTRIES)) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMallocHost(&h->lut_host, UST_LUT_WORDS * sizeof(uint32_t))) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMallocHost(&h->podlut_host, UST_PODLUT_ENTRIES)) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMalloc(&h->counters_dev, sizeof(ust_counters))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMallocHost(&h->counters_host, sizeof(ust_counters))) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMalloc(&h->xchg_dev, UST_V_LEN * sizeof(long long))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMalloc(&h->sp_count_dev, sizeof(long long))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMallocHost(&h->sp_count_host, sizeof(long long))) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = cudaMalloc(&h->lut_dev.p, UST_LUT_WORDS * sizeof(uint32_t))) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMalloc(&h->podlut_dev.p, UST_PODLUT_ENTRIES)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMallocHost(&h->lut_host.p, UST_LUT_WORDS * sizeof(uint32_t))) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = cudaMallocHost(&h->podlut_host.p, UST_PODLUT_ENTRIES)) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = cudaMalloc(&h->counters_dev.p, sizeof(ust_counters))) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMallocHost(&h->counters_host.p, sizeof(ust_counters))) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = cudaMalloc(&h->xchg_dev.p, UST_V_LEN * sizeof(long long))) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMalloc(&h->sp_count_dev.p, sizeof(long long))) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMallocHost(&h->sp_count_host.p, sizeof(long long))) != cudaSuccess) return bail("cudaMallocHost", e);
   if ((e = cudaMemset(h->xchg_dev, 0, UST_V_LEN * sizeof(long long))) != cudaSuccess) return bail("cudaMemset", e);
   if (const char* v = getenv("UST_PDL")) h->pdl = atoi(v) != 0;
   if (const char* v = getenv("UST_STATIC_PCT")) { h->static_pct = atoi(v); if (h->static_pct < 0) h->static_pct = 0; if (h->static_pct > 100) h->static_pct = 100; }
   h->stamps = getenv("UST_STAMPS") != nullptr;
   if (const char* v = getenv("UST_OVERLAP")) h->overlap_calls = atoi(v) != 0;
-  int rc = ust_stream_config(device, &h->num_sms, &h->stream_smem);
+  size_t stream_smem = 0;  // dynamic shared memory of the streaming kernel (largest variant)
+  int rc = ust_stream_config(device, &h->num_sms, &stream_smem);
   if (rc != 0 || h->num_sms < 1) {
     g_create_error = std::string("no sm_100a kernel image usable on this device: ") + cudaGetErrorString((cudaError_t)rc);
     ust_destroy(h);
@@ -621,39 +740,16 @@ int ust_create(ust_handle** out, int device) {
   return UST_OK;
 }
 
+// What needs an order: nothing in flight, the peers' mailboxes unmapped, the communicator gone. The handle's members
+// free its buffers, events and streams.
 void ust_destroy(ust_handle* h) {
   if (!h) return;
   if (h->device >= 0) cudaSetDevice(h->device);
-  if (h->stream_h2d) cudaStreamSynchronize(h->stream_h2d);
-  if (h->stream) cudaStreamSynchronize(h->stream);
-  if (h->stream_d2h) cudaStreamSynchronize(h->stream_d2h);
+  drain_streams(h);
   if (h->last_stream) cudaStreamSynchronize(h->last_stream);
   for (int r = 0; r < UST_MAX_WORLD; r++)
     if (h->mbox[r] && h->mbox[r] != h->mbox_own) cudaIpcCloseMemHandle(h->mbox[r]);
-  if (h->mbox_own) cudaFree(h->mbox_own);
   if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
-  if (h->ws) cudaFree(h->ws);
-  if (h->lut_dev) cudaFree(h->lut_dev);
-  if (h->podlut_dev) cudaFree(h->podlut_dev);
-  if (h->hist_dev) cudaFree(h->hist_dev);
-  if (h->lut_host) cudaFreeHost(h->lut_host);
-  if (h->podlut_host) cudaFreeHost(h->podlut_host);
-  if (h->counters_dev) cudaFree(h->counters_dev);
-  if (h->counters_host) cudaFreeHost(h->counters_host);
-  if (h->xchg_dev) cudaFree(h->xchg_dev);
-  if (h->sp_count_dev) cudaFree(h->sp_count_dev);
-  if (h->sp_count_host) cudaFreeHost(h->sp_count_host);
-  h->s_next_prev.release(); h->sp_next.release(); h->s_actions_prev.release(); h->sp_actions.release(); h->sp_blocks.release(); h->sp_idx.release();
-  if (h->ds_count_dev) cudaFree(h->ds_count_dev);
-  h->s_hot.release(); h->s_next.release(); h->s_outcome.release(); h->s_flags.release();
-  h->s_rev.release(); h->s_ds.release(); h->s_dsrev.release(); h->s_podoff.release(); h->s_dsdesired.release();
-  h->s_actions.release(); h->s_podflags.release(); h->s_podsum.release(); h->s_candtile[0].release(); h->s_candtile[1].release(); h->s_uid.release(); h->s_dsuid.release(); h->s_dsorder.release(); h->s_rev16.release(); h->s_ds8.release(); h->d_idx.release(); h->d_state.release(); h->d_flags.release(); h->d_rev.release(); h->d_ds.release(); h->sim_entered.release(); h->sim_wait.release(); h->sim_valid.release();
-  for (auto& ev : h->seg_done) if (ev) cudaEventDestroy(ev);
-  for (auto& ev : h->seg_up) if (ev) cudaEventDestroy(ev);
-  if (h->stream_h2d) cudaStreamDestroy(h->stream_h2d);
-  if (h->d2h_done) cudaEventDestroy(h->d2h_done);
-  if (h->stream_d2h) cudaStreamDestroy(h->stream_d2h);
-  if (h->stream) cudaStreamDestroy(h->stream);
   delete h;
 }
 
@@ -667,9 +763,7 @@ void ust_host_free(void* p) { if (p) cudaFreeHost(p); }
 void* ust_stream(ust_handle* h) { return h ? (void*)h->stream : nullptr; }
 
 int ust_sync(ust_handle* h) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   UST_CUDA(h, cudaSetDevice(h->device));
   cudaError_t e = cudaStreamSynchronize(h->stream);
   if (e == cudaSuccess && h->last_stream && h->last_stream != h->stream) e = cudaStreamSynchronize(h->last_stream);
@@ -682,12 +776,11 @@ int ust_apply_state_device(ust_handle* h, const ust_policy* policy, int64_t n_no
                            const int32_t* ds_rev, const ust_pods* pods, uint8_t* next_state, uint16_t* actions,
                            uint8_t* actuator_outcome, ust_counters* out_device, void* stream) {
   if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->chain_entry = true;  // the one entry point whose calls may overlap the previous call's tail (apply_device)
+  CallGuard call_guard(h, true);  // the one entry point whose calls may overlap the previous call's tail (apply_device)
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
   if (pods && (!pods->pod_off || pods->n_pods < 0 || (pods->n_pods > 0 && !pods->pod_flags)))
     return h->fail(UST_ERR_INVALID_ARGUMENT, "bad pod lists");
-  return apply_device(h, policy, n_nodes, state, flags, pod_rev, ds_idx, n_ds, ds_rev, pods ? pods->pod_off : nullptr,
+  return apply_device(h, true, policy, n_nodes, state, flags, pod_rev, ds_idx, n_ds, ds_rev, pods ? pods->pod_off : nullptr,
                       pods ? pods->pod_flags : nullptr, pods ? pods->n_pods : 0, next_state, actions, actuator_outcome,
                       out_device, st);
 }
@@ -696,60 +789,26 @@ int ust_apply_state(ust_handle* h, const ust_policy* policy, int64_t n, const ui
                     const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds, const int32_t* ds_rev,
                     const ust_pods* pods, uint8_t* next_state, uint16_t* actions, uint8_t* actuator_outcome,
                     ust_counters* out) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   if (n < 0 || (n > 0 && (!state || !flags || !pod_rev || !ds_idx || !next_state || !actions)))
     return h->fail(UST_ERR_NIL_STATE, "currentState should not be empty");
   if (n_ds < 0 || (n_ds > 0 && !ds_rev)) return h->fail(UST_ERR_INVALID_ARGUMENT, "bad DaemonSet table");
   if (pods && (!pods->pod_off || pods->n_pods < 0 || (pods->n_pods > 0 && !pods->pod_flags)))
     return h->fail(UST_ERR_INVALID_ARGUMENT, "bad pod lists");
   if (pods) { int prc = check_pod_offsets_host(h, n, pods->pod_off, pods->n_pods); if (prc) return prc; }
-  UST_CUDA(h, cudaSetDevice(h->device));
-  StreamDrain drain(h);
-  cudaStream_t st = h->stream;
-  const size_t N = (size_t)n;
-  UST_CUDA(h, h->s_hot.reserve(N + 16));
-  UST_CUDA(h, h->s_flags.reserve(N + 4));
-  UST_CUDA(h, h->s_rev.reserve(N + 4));
-  UST_CUDA(h, h->s_ds.reserve(N + 4));
-  UST_CUDA(h, h->s_next.reserve(N + 16));
-  UST_CUDA(h, h->s_actions.reserve(N + 8));
-  UST_CUDA(h, h->s_dsrev.reserve((size_t)n_ds + 1));
-  if (actuator_outcome) UST_CUDA(h, h->s_outcome.reserve(N + 16));
-  if (pods) {
-    UST_CUDA(h, h->s_podoff.reserve(N + 1));
-    UST_CUDA(h, h->s_podflags.reserve((size_t)pods->n_pods + 8));
-  }
-  if (n_ds) UST_CUDA(h, cudaMemcpyAsync(h->s_dsrev.p, ds_rev, (size_t)n_ds * 4, cudaMemcpyHostToDevice, st));
-  h->resident_n = -1;
-  h->outputs_resident = false;
-  auto keep = [&](int rc) {  // the uploaded snapshot stays usable unless the call itself failed (not the policy / the data)
-    if (rc != UST_ERR_CUDA && rc != UST_ERR_INVALID_ARGUMENT && rc != UST_ERR_COMM && rc != UST_ERR_NIL_STATE && !pods) { h->resident_n = n; h->resident_n_ds = n_ds; h->outputs_resident = true; }
-    return rc;
-  };
-  if (!pods && n >= (1 << 19))
-    return keep(apply_pipelined(h, policy, n, state, flags, pod_rev, ds_idx, n_ds, next_state, actions, actuator_outcome, out));
-  if (N) {
-    UST_CUDA(h, cudaMemcpyAsync(h->s_hot.p, state, N, cudaMemcpyHostToDevice, st));
-    UST_CUDA(h, cudaMemcpyAsync(h->s_flags.p, flags, N * 4, cudaMemcpyHostToDevice, st));
-    UST_CUDA(h, cudaMemcpyAsync(h->s_rev.p, pod_rev, N * 4, cudaMemcpyHostToDevice, st));
-    UST_CUDA(h, cudaMemcpyAsync(h->s_ds.p, ds_idx, N * 4, cudaMemcpyHostToDevice, st));
-  }
-  if (pods) {
-    UST_CUDA(h, cudaMemcpyAsync(h->s_podoff.p, pods->pod_off, (N + 1) * 4, cudaMemcpyHostToDevice, st));
-    if (pods->n_pods) UST_CUDA(h, cudaMemcpyAsync(h->s_podflags.p, pods->pod_flags, (size_t)pods->n_pods * 2, cudaMemcpyHostToDevice, st));
-  }
-  int rc = apply_device(h, policy, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p,
-                        pods ? h->s_podoff.p : nullptr, pods ? h->s_podflags.p : nullptr, pods ? pods->n_pods : 0, h->s_next.p,
-                        h->s_actions.p, actuator_outcome ? h->s_outcome.p : nullptr, nullptr, st);
-  if (rc) return rc;
-  if (N) {
-    UST_CUDA(h, cudaMemcpyAsync(next_state, h->s_next.p, N, cudaMemcpyDeviceToHost, st));
-    UST_CUDA(h, cudaMemcpyAsync(actions, h->s_actions.p, N * 2, cudaMemcpyDeviceToHost, st));
-    if (actuator_outcome) UST_CUDA(h, cudaMemcpyAsync(actuator_outcome, h->s_outcome.p, N, cudaMemcpyDeviceToHost, st));
-  }
-  return keep(finish_with_counters(h, st, out));
+  const HostNodes nodes{h, false, state, flags, pod_rev, ds_idx, nullptr, nullptr};
+  return apply_host(h, policy, n, nodes, n_ds, ds_rev, pods, next_state, actions, actuator_outcome, out);
+}
+
+int ust_apply_state_packed(ust_handle* h, const ust_policy* policy, int64_t n, const uint8_t* state, const uint32_t* flags,
+                           const uint16_t* pod_rev16, const int8_t* ds_idx8, int32_t n_ds, const int32_t* ds_rev,
+                           uint8_t* next_state, uint16_t* actions, uint8_t* actuator_outcome, ust_counters* out) {
+  UST_ENTER(h);
+  if (n < 0 || (n > 0 && (!state || !flags || !pod_rev16 || !ds_idx8 || !next_state || !actions)))
+    return h->fail(UST_ERR_NIL_STATE, "currentState should not be empty");
+  if (n_ds < 0 || n_ds > 127 || (n_ds > 0 && !ds_rev)) return h->fail(UST_ERR_INVALID_ARGUMENT, "bad DaemonSet table (the packed format holds at most 127 DaemonSets)");
+  const HostNodes nodes{h, true, state, flags, nullptr, nullptr, pod_rev16, ds_idx8};
+  return apply_host(h, policy, n, nodes, n_ds, ds_rev, nullptr, next_state, actions, actuator_outcome, out);
 }
 
 // ust_apply_state_delta and ust_apply_state_delta_sparse: scatter the re-encoded nodes into the resident snapshot,
@@ -786,8 +845,7 @@ static int delta_common(ust_handle* h, const ust_policy* policy, int64_t n_chang
     UST_CUDA(h, h->sp_next.reserve((size_t)max_out + 16));
     UST_CUDA(h, h->sp_actions.reserve((size_t)max_out + 8));
   }
-  h->resident_n = -1;  // until the patched snapshot has been evaluated
-  h->outputs_resident = false;
+  drop_resident(h);  // until the patched snapshot has been evaluated
   if (n_ds) UST_CUDA(h, cudaMemcpyAsync(h->s_dsrev.p, ds_rev, (size_t)n_ds * 4, cudaMemcpyHostToDevice, st));
   if (M) {
     static_assert(sizeof(long long) == sizeof(int64_t), "index width");
@@ -805,15 +863,11 @@ static int delta_common(ust_handle* h, const ust_policy* policy, int64_t n_chang
     std::swap(h->s_next, h->s_next_prev);
     std::swap(h->s_actions, h->s_actions_prev);
   }
-  int rc = apply_device(h, policy, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p, nullptr, nullptr, 0,
-                        h->s_next.p, h->s_actions.p, actuator_outcome ? h->s_outcome.p : nullptr, nullptr, st);
+  int rc = apply_device(h, false, policy, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p, nullptr, nullptr,
+                        0, h->s_next.p, h->s_actions.p, actuator_outcome ? h->s_outcome.p : nullptr, nullptr, st);
   if (rc) return rc;
   if (!sparse) {
-    if (N) {
-      UST_CUDA(h, cudaMemcpyAsync(next_state, h->s_next.p, N, cudaMemcpyDeviceToHost, st));
-      UST_CUDA(h, cudaMemcpyAsync(actions, h->s_actions.p, N * 2, cudaMemcpyDeviceToHost, st));
-      if (actuator_outcome) UST_CUDA(h, cudaMemcpyAsync(actuator_outcome, h->s_outcome.p, N, cudaMemcpyDeviceToHost, st));
-    }
+    if ((rc = download_outputs(h, 0, N, next_state, actions, actuator_outcome, st))) return rc;
   } else {
     int e = ust_launch_diff((long long)n, h->s_next.p, h->s_actions.p, h->s_next_prev.p, h->s_actions_prev.p, h->sp_blocks.p,
                             h->sp_count_dev, (long long)max_out, h->sp_idx.p, h->sp_next.p, h->sp_actions.p, st);
@@ -829,8 +883,7 @@ static int delta_common(ust_handle* h, const ust_policy* policy, int64_t n_chang
       UST_CUDA(h, cudaMemcpyAsync(actions, h->sp_actions.p, (size_t)cnt * 2, cudaMemcpyDeviceToHost, st));
     }
   }
-  rc = finish_with_counters(h, st, out);
-  if (rc != UST_ERR_CUDA && rc != UST_ERR_COMM) { h->resident_n = n; h->resident_n_ds = n_ds; h->outputs_resident = true; }
+  rc = keep_resident(h, finish_with_counters(h, st, out), n, n_ds);
   if (sparse && (rc == UST_OK) && *n_out > max_out)
     return h->fail(UST_ERR_TRUNCATED, "%lld outputs changed, the caller's arrays hold %lld: fetch them with ust_fetch_outputs", (long long)*n_out, (long long)max_out);
   return rc;
@@ -840,9 +893,7 @@ int ust_apply_state_delta(ust_handle* h, const ust_policy* policy, int64_t n_cha
                           const uint32_t* flags, const int32_t* pod_rev, const int32_t* ds_idx, int32_t n_ds,
                           const int32_t* ds_rev, uint8_t* next_state, uint16_t* actions, uint8_t* actuator_outcome,
                           ust_counters* out) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   return delta_common(h, policy, n_changed, idx, state, flags, pod_rev, ds_idx, n_ds, ds_rev, false, next_state, actions,
                       actuator_outcome, 0, nullptr, nullptr, out);
 }
@@ -851,80 +902,20 @@ int ust_apply_state_delta_sparse(ust_handle* h, const ust_policy* policy, int64_
                                  const uint8_t* state, const uint32_t* flags, const int32_t* pod_rev, const int32_t* ds_idx,
                                  int32_t n_ds, const int32_t* ds_rev, int64_t max_out, int64_t* out_idx,
                                  uint8_t* out_next_state, uint16_t* out_actions, int64_t* n_out, ust_counters* out) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   return delta_common(h, policy, n_changed, idx, state, flags, pod_rev, ds_idx, n_ds, ds_rev, true, out_next_state, out_actions,
                       nullptr, max_out, out_idx, n_out, out);
 }
 
 int ust_fetch_outputs(ust_handle* h, uint8_t* next_state, uint16_t* actions) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   if (h->resident_n < 0 || !h->outputs_resident) return h->fail(UST_ERR_INVALID_ARGUMENT, "no resident outputs");
   if (h->resident_n > 0 && (!next_state || !actions)) return h->fail(UST_ERR_INVALID_ARGUMENT, "bad arguments");
   UST_CUDA(h, cudaSetDevice(h->device));
-  const size_t N = (size_t)h->resident_n;
-  if (N) {
-    UST_CUDA(h, cudaMemcpyAsync(next_state, h->s_next.p, N, cudaMemcpyDeviceToHost, h->stream));
-    UST_CUDA(h, cudaMemcpyAsync(actions, h->s_actions.p, N * 2, cudaMemcpyDeviceToHost, h->stream));
-  }
+  int rc = download_outputs(h, 0, (size_t)h->resident_n, next_state, actions, nullptr, h->stream);
+  if (rc) return rc;
   UST_CUDA(h, cudaStreamSynchronize(h->stream));
   return UST_OK;
-}
-
-int ust_apply_state_packed(ust_handle* h, const ust_policy* policy, int64_t n, const uint8_t* state, const uint32_t* flags,
-                           const uint16_t* pod_rev16, const int8_t* ds_idx8, int32_t n_ds, const int32_t* ds_rev,
-                           uint8_t* next_state, uint16_t* actions, uint8_t* actuator_outcome, ust_counters* out) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
-  if (n < 0 || (n > 0 && (!state || !flags || !pod_rev16 || !ds_idx8 || !next_state || !actions)))
-    return h->fail(UST_ERR_NIL_STATE, "currentState should not be empty");
-  if (n_ds < 0 || n_ds > 127 || (n_ds > 0 && !ds_rev)) return h->fail(UST_ERR_INVALID_ARGUMENT, "bad DaemonSet table (the packed format holds at most 127 DaemonSets)");
-  UST_CUDA(h, cudaSetDevice(h->device));
-  StreamDrain drain(h);
-  cudaStream_t st = h->stream;
-  const size_t N = (size_t)n;
-  UST_CUDA(h, h->s_hot.reserve(N + 16));
-  UST_CUDA(h, h->s_flags.reserve(N + 4));
-  UST_CUDA(h, h->s_rev.reserve(N + 4));
-  UST_CUDA(h, h->s_ds.reserve(N + 4));
-  UST_CUDA(h, h->s_rev16.reserve(N + 8));
-  UST_CUDA(h, h->s_ds8.reserve(N + 16));
-  UST_CUDA(h, h->s_next.reserve(N + 16));
-  UST_CUDA(h, h->s_actions.reserve(N + 8));
-  UST_CUDA(h, h->s_dsrev.reserve((size_t)n_ds + 1));
-  if (actuator_outcome) UST_CUDA(h, h->s_outcome.reserve(N + 16));
-  if (n_ds) UST_CUDA(h, cudaMemcpyAsync(h->s_dsrev.p, ds_rev, (size_t)n_ds * 4, cudaMemcpyHostToDevice, st));
-  h->resident_n = -1;
-  h->outputs_resident = false;
-  auto keep = [&](int rc) {
-    if (rc != UST_ERR_CUDA && rc != UST_ERR_INVALID_ARGUMENT && rc != UST_ERR_COMM && rc != UST_ERR_NIL_STATE) { h->resident_n = n; h->resident_n_ds = n_ds; h->outputs_resident = true; }
-    return rc;
-  };
-  if (n >= (1 << 19))
-    return keep(apply_pipelined(h, policy, n, state, flags, nullptr, nullptr, n_ds, next_state, actions, actuator_outcome, out,
-                                pod_rev16, ds_idx8));
-  if (N) {
-    UST_CUDA(h, cudaMemcpyAsync(h->s_hot.p, state, N, cudaMemcpyHostToDevice, st));
-    UST_CUDA(h, cudaMemcpyAsync(h->s_flags.p, flags, N * 4, cudaMemcpyHostToDevice, st));
-    UST_CUDA(h, cudaMemcpyAsync(h->s_rev16.p, pod_rev16, N * 2, cudaMemcpyHostToDevice, st));
-    UST_CUDA(h, cudaMemcpyAsync(h->s_ds8.p, ds_idx8, N, cudaMemcpyHostToDevice, st));
-    int we = ust_launch_widen((long long)n, h->s_rev16.p, h->s_ds8.p, h->s_rev.p, h->s_ds.p, 4 * h->num_sms, st);
-    if (we) return h->fail(UST_ERR_CUDA, "widen kernel launch failed: %s", cudaGetErrorString((cudaError_t)we));
-    h->launches += 1;
-  }
-  int rc = apply_device(h, policy, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, n_ds, h->s_dsrev.p, nullptr, nullptr, 0,
-                        h->s_next.p, h->s_actions.p, actuator_outcome ? h->s_outcome.p : nullptr, nullptr, st);
-  if (rc) return rc;
-  if (N) {
-    UST_CUDA(h, cudaMemcpyAsync(next_state, h->s_next.p, N, cudaMemcpyDeviceToHost, st));
-    UST_CUDA(h, cudaMemcpyAsync(actions, h->s_actions.p, N * 2, cudaMemcpyDeviceToHost, st));
-    if (actuator_outcome) UST_CUDA(h, cudaMemcpyAsync(actuator_outcome, h->s_outcome.p, N, cudaMemcpyDeviceToHost, st));
-  }
-  return keep(finish_with_counters(h, st, out));
 }
 
 static int simulate_common(ust_handle* h, const ust_policy* policy, const ust_sim_options* opt, int32_t steps, ust_counters* history,
@@ -945,13 +936,8 @@ static int simulate_common(ust_handle* h, const ust_policy* policy, const ust_si
   cudaStream_t st = h->stream;
   const size_t N = (size_t)n;
   UST_CUDA(h, h->s_outcome.reserve(N + 16));
-  if ((size_t)steps + 1 > h->hist_cap) {
-    if (h->hist_dev) cudaFree(h->hist_dev);
-    h->hist_cap = (size_t)steps + 64;
-    UST_CUDA(h, cudaMalloc(&h->hist_dev, h->hist_cap * sizeof(ust_counters)));
-  }
-  h->resident_n = -1;
-  h->outputs_resident = false;
+  if ((size_t)steps + 1 > h->hist.cap) UST_CUDA(h, h->hist.resize((size_t)steps + 64));
+  drop_resident(h);
   int grid = 8 * h->num_sms;
   UstSimParams sp;
   memset(&sp, 0, sizeof(sp));
@@ -966,18 +952,18 @@ static int simulate_common(ust_handle* h, const ust_policy* policy, const ust_si
     h->launches += 1;
   }
   for (int32_t k = 0; k < steps; k++) {
-    int rc = apply_device(h, policy ? &pol : nullptr, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, h->resident_n_ds,
-                          h->s_dsrev.p, nullptr, nullptr, 0, h->s_next.p, h->s_actions.p, h->s_outcome.p, h->hist_dev + k, st);
+    int rc = apply_device(h, false, policy ? &pol : nullptr, n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, h->resident_n_ds,
+                          h->s_dsrev.p, nullptr, nullptr, 0, h->s_next.p, h->s_actions.p, h->s_outcome.p, h->hist.p + k, st);
     if (rc) return rc;
     sp.now = (long long)k * sp.dt;
     int e = ust_launch_feedback(n, h->s_hot.p, h->s_flags.p, h->s_rev.p, h->s_ds.p, h->resident_n_ds, h->s_dsrev.p, h->s_next.p,
-                                h->s_actions.p, h->s_outcome.p, h->hist_dev + k, sp, h->sim_entered.p, h->sim_wait.p, h->sim_valid.p,
+                                h->s_actions.p, h->s_outcome.p, h->hist.p + k, sp, h->sim_entered.p, h->sim_wait.p, h->sim_valid.p,
                                 grid, st);
     if (e) return h->fail(UST_ERR_CUDA, "feedback kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
     h->launches += 1;
   }
   std::vector<ust_counters> hist((size_t)steps);
-  if (steps) UST_CUDA(h, cudaMemcpyAsync(hist.data(), h->hist_dev, (size_t)steps * sizeof(ust_counters), cudaMemcpyDeviceToHost, st));
+  if (steps) UST_CUDA(h, cudaMemcpyAsync(hist.data(), h->hist.p, (size_t)steps * sizeof(ust_counters), cudaMemcpyDeviceToHost, st));
   if (N && final_state) UST_CUDA(h, cudaMemcpyAsync(final_state, h->s_hot.p, N, cudaMemcpyDeviceToHost, st));
   if (N && final_flags) UST_CUDA(h, cudaMemcpyAsync(final_flags, h->s_flags.p, N * 4, cudaMemcpyDeviceToHost, st));
   if (N && final_pod_rev) UST_CUDA(h, cudaMemcpyAsync(final_pod_rev, h->s_rev.p, N * 4, cudaMemcpyDeviceToHost, st));
@@ -997,54 +983,38 @@ static int simulate_common(ust_handle* h, const ust_policy* policy, const ust_si
 
 int ust_simulate_rollout(ust_handle* h, const ust_policy* policy, int32_t steps, ust_counters* history, uint8_t* final_state,
                          uint32_t* final_flags, int32_t* final_pod_rev, int32_t* steps_done) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   return simulate_common(h, policy, nullptr, steps, history, final_state, final_flags, final_pod_rev, steps_done);
 }
 
 int ust_simulate_rollout_timed(ust_handle* h, const ust_policy* policy, const ust_sim_options* options, int32_t steps,
                                ust_counters* history, uint8_t* final_state, uint32_t* final_flags, int32_t* final_pod_rev,
                                int32_t* steps_done) {
-  if (!h || !options) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  if (!options) return UST_ERR_INVALID_ARGUMENT;
+  UST_ENTER(h);
   return simulate_common(h, policy, options, steps, history, final_state, final_flags, final_pod_rev, steps_done);
 }
 
 int ust_build_state(ust_handle* h, int64_t n_pods, const uint8_t* state, const int32_t* ds_idx, int32_t n_ds,
                     const int32_t* ds_desired, ust_counters* out) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   if (n_pods < 0 || (n_pods > 0 && (!state || !ds_idx)) || n_ds < 0 || (n_ds > 0 && !ds_desired))
     return h->fail(UST_ERR_INVALID_ARGUMENT, "bad arguments");
-  h->resident_n = -1;  // shares the staging arrays
-  h->outputs_resident = false;
+  drop_resident(h);  // shares the staging arrays
   UST_CUDA(h, cudaSetDevice(h->device));
   StreamDrain drain(h);
   cudaStream_t st = h->stream;
   const size_t N = (size_t)n_pods;
-  UST_CUDA(h, h->s_hot.reserve(N + 16));
-  UST_CUDA(h, h->s_ds.reserve(N + 4));
-  UST_CUDA(h, h->s_dsdesired.reserve((size_t)n_ds + 1));
-  if ((size_t)n_ds + 1 > h->ds_count_cap) {
-    if (h->ds_count_dev) cudaFree(h->ds_count_dev);
-    h->ds_count_cap = (size_t)n_ds + 64;
-    UST_CUDA(h, cudaMalloc(&h->ds_count_dev, h->ds_count_cap * sizeof(unsigned long long)));
-    UST_CUDA(h, cudaMemsetAsync(h->ds_count_dev, 0, h->ds_count_cap * sizeof(unsigned long long), st));
-  }
-  if (h->ws_dirty) { UST_CUDA(h, cudaMemsetAsync(h->ws, 0, sizeof(UstWorkspace), st)); h->ws_dirty = false; }
+  int rc = stage_build_state(h, N, n_ds, st);
+  if (rc) return rc;
   if (N) {
     UST_CUDA(h, cudaMemcpyAsync(h->s_hot.p, state, N, cudaMemcpyHostToDevice, st));
     UST_CUDA(h, cudaMemcpyAsync(h->s_ds.p, ds_idx, N * 4, cudaMemcpyHostToDevice, st));
   }
   if (n_ds) UST_CUDA(h, cudaMemcpyAsync(h->s_dsdesired.p, ds_desired, (size_t)n_ds * 4, cudaMemcpyHostToDevice, st));
-  int64_t grid = (n_pods + 1023) / 1024;  // 256 threads x 4 pods per iteration
-  if (grid < 1) grid = 1;
-  if (grid > 8 * h->num_sms) grid = 8 * h->num_sms;
   h->ws_dirty = true;
-  int e = ust_launch_build_state(n_pods, h->s_hot.p, h->s_ds.p, n_ds, h->s_dsdesired.p, h->ds_count_dev, h->ws, h->counters_dev, (int)grid, st);
+  int e = ust_launch_build_state(n_pods, h->s_hot.p, h->s_ds.p, n_ds, h->s_dsdesired.p, h->ds_count.p, h->ws, h->counters_dev,
+                                 build_state_grid(h, n_pods), st);
   if (e) return h->fail(UST_ERR_CUDA, "build-state kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
   h->ws_dirty = false;
   h->launches += 2;
@@ -1053,9 +1023,7 @@ int ust_build_state(ust_handle* h, int64_t n_pods, const uint8_t* state, const i
 
 int ust_build_state_uids(ust_handle* h, int64_t n_pods, const uint8_t* state, const uint64_t* owner_uid, int32_t n_ds,
                          const uint64_t* ds_uid, const int32_t* ds_desired, int32_t* ds_idx_out, ust_counters* out) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   if (n_pods < 0 || (n_pods > 0 && (!state || !owner_uid || !ds_idx_out)) || n_ds < 0 || (n_ds > 0 && (!ds_uid || !ds_desired)))
     return h->fail(UST_ERR_INVALID_ARGUMENT, "bad arguments");
   // the DaemonSet map is keyed by UID (common_manager.go:181-185): an open-addressing table at load factor <= 1/4
@@ -1074,25 +1042,16 @@ int ust_build_state_uids(ust_handle* h, int64_t n_pods, const uint8_t* state, co
     }
     tab[2 * s] = x; tab[2 * s + 1] = y; tab_idx[s] = d;
   }
-  h->resident_n = -1;  // shares the staging arrays
-  h->outputs_resident = false;
+  drop_resident(h);  // shares the staging arrays
   UST_CUDA(h, cudaSetDevice(h->device));
   StreamDrain drain(h);
   cudaStream_t st = h->stream;
   const size_t N = (size_t)n_pods;
-  UST_CUDA(h, h->s_hot.reserve(N + 16));
-  UST_CUDA(h, h->s_ds.reserve(N + 4));
   UST_CUDA(h, h->s_uid.reserve(2 * N + 2));
   UST_CUDA(h, h->s_dsuid.reserve(2 * slots));
   UST_CUDA(h, h->s_dsorder.reserve(slots));
-  UST_CUDA(h, h->s_dsdesired.reserve((size_t)n_ds + 1));
-  if ((size_t)n_ds + 1 > h->ds_count_cap) {
-    if (h->ds_count_dev) cudaFree(h->ds_count_dev);
-    h->ds_count_cap = (size_t)n_ds + 64;
-    UST_CUDA(h, cudaMalloc(&h->ds_count_dev, h->ds_count_cap * sizeof(unsigned long long)));
-    UST_CUDA(h, cudaMemsetAsync(h->ds_count_dev, 0, h->ds_count_cap * sizeof(unsigned long long), st));
-  }
-  if (h->ws_dirty) { UST_CUDA(h, cudaMemsetAsync(h->ws, 0, sizeof(UstWorkspace), st)); h->ws_dirty = false; }
+  int rc = stage_build_state(h, N, n_ds, st);
+  if (rc) return rc;
   if (N) {
     UST_CUDA(h, cudaMemcpyAsync(h->s_hot.p, state, N, cudaMemcpyHostToDevice, st));
     UST_CUDA(h, cudaMemcpyAsync(h->s_uid.p, owner_uid, N * 16, cudaMemcpyHostToDevice, st));
@@ -1100,12 +1059,10 @@ int ust_build_state_uids(ust_handle* h, int64_t n_pods, const uint8_t* state, co
   UST_CUDA(h, cudaMemcpyAsync(h->s_dsuid.p, tab.data(), slots * 16, cudaMemcpyHostToDevice, st));
   UST_CUDA(h, cudaMemcpyAsync(h->s_dsorder.p, tab_idx.data(), slots * 4, cudaMemcpyHostToDevice, st));
   if (n_ds) UST_CUDA(h, cudaMemcpyAsync(h->s_dsdesired.p, ds_desired, (size_t)n_ds * 4, cudaMemcpyHostToDevice, st));
-  int64_t grid = (n_pods + 1023) / 1024;  // 256 threads x 4 pods per iteration
-  if (grid < 1) grid = 1;
-  if (grid > 8 * h->num_sms) grid = 8 * h->num_sms;
   h->ws_dirty = true;
   int e = ust_launch_build_state_uids(n_pods, h->s_hot.p, h->s_uid.p, n_ds, h->s_dsuid.p, h->s_dsorder.p, (int)slots,
-                                      h->s_dsdesired.p, h->s_ds.p, h->ds_count_dev, h->ws, h->counters_dev, (int)grid, st);
+                                      h->s_dsdesired.p, h->s_ds.p, h->ds_count.p, h->ws, h->counters_dev,
+                                      build_state_grid(h, n_pods), st);
   if (e) return h->fail(UST_ERR_CUDA, "build-state kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
   h->ws_dirty = false;
   h->launches += 2;
@@ -1145,9 +1102,8 @@ long long ust_debug_relaxed_calls(ust_handle* h) { return h ? (long long)h->rela
 
 // diagnostics (not in include/ust.h): %globaltimer stamps taken by CTA 0 of the last fused launch
 int ust_debug_stamps(ust_handle* h, unsigned long long* out, int n_ctas) {
-  if (!h || !out || n_ctas < 1 || n_ctas > UST_MAX_CTAS) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  if (!out || n_ctas < 1 || n_ctas > UST_MAX_CTAS) return UST_ERR_INVALID_ARGUMENT;
+  UST_ENTER(h);
   UST_CUDA(h, cudaSetDevice(h->device));
   UST_CUDA(h, cudaDeviceSynchronize());
   UST_CUDA(h, cudaMemcpy(out, h->ws->dbg, (size_t)n_ctas * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
@@ -1168,9 +1124,7 @@ int ust_get_unique_id(void* out_bytes) {
 }
 
 int ust_comm_init(ust_handle* h, int rank, int world_size, const void* unique_id_bytes) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   if (world_size < 1 || world_size > UST_MAX_WORLD || rank < 0 || rank >= world_size)
     return h->fail(UST_ERR_INVALID_ARGUMENT, "world size must be 1..%d", UST_MAX_WORLD);
   if (world_size == 1) { h->rank = 0; h->world = 1; return UST_OK; }
@@ -1192,7 +1146,7 @@ int ust_comm_init(ust_handle* h, int rank, int world_size, const void* unique_id
   h->mbox_ready = false;
   do {
     if (!g_nccl.AllGather) break;
-    if (cudaMalloc(&h->mbox_own, sizeof(UstMailbox)) != cudaSuccess) break;
+    if (cudaMalloc(&h->mbox_own.p, sizeof(UstMailbox)) != cudaSuccess) break;
     if (cudaMemset(h->mbox_own, 0, sizeof(UstMailbox)) != cudaSuccess) break;
     cudaIpcMemHandle_t mine;
     if (cudaIpcGetMemHandle(&mine, h->mbox_own) != cudaSuccess) { cudaGetLastError(); break; }
@@ -1219,9 +1173,7 @@ int ust_comm_init(ust_handle* h, int rank, int world_size, const void* unique_id
 }
 
 int ust_comm_set_mode(ust_handle* h, int mode) {
-  if (!h) return UST_ERR_INVALID_ARGUMENT;
-  std::lock_guard<std::mutex> g(h->mu);
-  h->prev_n = -1;  // whatever this entry point enqueues sits between two device calls: they keep the strict order
+  UST_ENTER(h);
   if (mode != 0 && mode != 1) return h->fail(UST_ERR_INVALID_ARGUMENT, "unknown exchange mode %d", mode);
   if (mode == 1 && !(h->world > 1 && h->mbox_ready))
     return h->fail(UST_ERR_COMM, "fused exchange unavailable: peer mailboxes could not be mapped (CUDA IPC)");
